@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the CPU restatement of the reference path, host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also store what the last timed step computed
 
 A "step" is one pass of the hot path over one batch of synthetic requests.  Workload at every N: BASELINE config 2 —
 16-route GET table, 256-byte JSON struct body, 1 Mi requests per GPU (weak scaling: each rank serves its own
@@ -182,6 +183,37 @@ class ClockSampler:
                 pass
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons),
                 "samples": len(sm), "source": "nvidia-smi"}
+
+
+DUMP_ROWS = 16384  # responses --dump-outputs stores byte for byte: 16 Ki 528-byte slots as float32 are 35 MB
+
+
+def dump_outputs(path, n, width, slots, resp):
+    """--dump-outputs: what the resident path handed its caller in the last timed step (`slots` = (out, out_len, meta) of
+    the slot layout, else the packed `resp`), for comparing two builds output for output.  A fixed, seeded sample of
+    DUMP_ROWS requests (all of them when there are fewer): their response bytes (zero past each response's end), lengths
+    and meta words, in the same form for both layouts.  float32 holds every byte and length exactly, float64 every uint32
+    meta word and request index."""
+    import torch
+    k = min(n, DUMP_ROWS)
+    idx = np.sort(np.random.default_rng(synth.SEED).choice(n, k, replace=False))
+    i = torch.from_numpy(idx).to(resp.out.device)
+    if slots is not None:
+        s_out, s_len, s_meta = slots
+        buf, start, length, meta = s_out, i * width, s_len[i].long(), s_meta[i]
+    else:
+        off = resp.out_off.long() & 0xFFFFFFFF
+        buf, start, length, meta = resp.out, off[i], off[i + 1] - off[i], resp.meta[i]
+    assert bool((length <= width).all()), "a response longer than the dump's row width"
+    col = torch.arange(width, device=buf.device)
+    keep = col < length[:, None]
+    rows = torch.where(keep, buf[torch.where(keep, start[:, None] + col, 0)], 0)
+    arrays = {"request_index": idx.astype(np.float64), "response_bytes": rows.cpu().numpy().astype(np.float32),
+              "response_len": length.cpu().numpy().astype(np.float32),
+              "meta": (meta.long() & 0xFFFFFFFF).cpu().numpy().astype(np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def bind_to_gpu_numa(device: int):
@@ -674,7 +706,14 @@ def main():
                          "(gofr_serve_device_slots)")
     ap.add_argument("--workload", default="config2", choices=["config2", "config3", "config4", "config5", "proto", "reqlog", "http"],
                     help="config2 is the BASELINE metric line; the others are secondary measurements (resident only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's shard; a seeded sample of "
+                         "%d responses, their lengths and meta words) as DIR/<name>.npy in float32 / float64" % DUMP_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.workload != "config2"):
+        ap.error("--dump-outputs stores the outputs of the config-2 headline path only")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -766,6 +805,8 @@ def main():
     per_launch_ms = kernel_ms / max(kernel_launches, 1)
     achieved = algo_bytes / (per_launch_ms / 1e3) / 1e9
     peak, peak_src = hbm_peak()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, slot, (s_out, s_len, s_meta) if args.layout == "slots" else None, resp)
 
     # the other layout, measured the same way (reported beside the headline number, not instead of it)
     alt = None
