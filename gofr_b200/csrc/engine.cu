@@ -139,9 +139,8 @@ static void register_engine(int device, int delta) {
 // registers) is asked for (GOFR_SLOT_CTAS=4, gofr_engine_slot_ctas).  For a short while the wide instance was the default
 // for one-shape fast-path tables — it measured 4 % faster than the "5-CTA" instance on config 2 — until it turned out that
 // the 5-CTA instances had been resident 4 per SM (DESIGN.md section 4e): with the fifth CTA back they are 7.5 % faster than
-// the wide one on the same table (0.2737 against 0.2959 ms).  image_wants_wide_slots (table_build.cpp) still tells which
-// tables the wide instance was meant for.
-static bool choose_slot_residency(const std::vector<uint8_t>&, const ImageHeader&) {
+// the wide one on the same table (0.2737 against 0.2959 ms).
+static bool choose_slot_residency() {
     if (const char* v = getenv("GOFR_SLOT_CTAS")) return atoi(v) == kServeCtasWide;
     return false;
 }
@@ -214,7 +213,7 @@ static int engine_init(gofr_engine* e, const std::vector<uint8_t>& img, int devi
     if (w_in_per < in_per) w_in_per = in_per;
     int rc = configure_geometry(e, in_per, w_in_per);
     if (rc != GOFR_OK) return rc;
-    e->slots_wide = choose_slot_residency(img, e->hdr);
+    e->slots_wide = choose_slot_residency();
     for (uint32_t k = 0; k < e->hdr.n_progs; k++)
         e->has_values |= (reinterpret_cast<const ProgRec*>(img.data() + e->hdr.progs_off)[k].flags & PF_VALUES) != 0;
     for (auto& s : e->slots) {
@@ -317,6 +316,87 @@ static int next_epoch(gofr_engine* e, uint32_t* out) {
     return GOFR_OK;
 }
 
+// Look-back state of the resident calls for `tiles` tiles.  cudaFree synchronises, so no earlier launch still uses the
+// old buffer.  Called with the engine lock held.
+static int grow_state(gofr_engine* e, size_t tiles) {
+    if (tiles <= e->state_tiles) return GOFR_OK;
+    cudaFree(e->d_state);
+    e->d_state = nullptr;
+    e->state_tiles = 0;
+    CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
+    CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
+    e->state_tiles = tiles;
+    return GOFR_OK;
+}
+
+// Bind scratch of the resident serve calls for n requests; nothing for a table without Bind-echo routes.
+static int grow_bind(gofr_engine* e, uint32_t n) {
+    const size_t need = (size_t)n * e->hdr.bind_row_words * 4;
+    if (need <= e->bind_cap) return GOFR_OK;
+    cudaFree(e->d_bind);
+    e->d_bind = nullptr;
+    e->bind_cap = 0;
+    CUDA_TRY(cudaMalloc(&e->d_bind, need + need / 4 + 256));
+    e->bind_cap = need + need / 4;
+    return GOFR_OK;
+}
+
+// Grid of a look-back kernel: its resident grid shared with the other engines on the device (see engines_on_device),
+// and no more CTAs than tiles.
+static int lookback_grid(gofr_engine* e, int grid, size_t tiles) {
+    return (int)std::min<size_t>((size_t)std::max(1, grid / engines_on_device(e->device)), tiles);
+}
+
+// A kernel's resident grid, asked from the occupancy calculator on first use.
+static int lazy_grid(gofr_engine* e, int* grid, int (*max_grid)(int), const char* what) {
+    if (*grid <= 0) {
+        *grid = max_grid(e->device);
+        if (*grid <= 0) { set_last_error("%s kernel cannot be resident", what); return GOFR_ERR_CUDA; }
+    }
+    return GOFR_OK;
+}
+
+// Enqueues one kernel on `st` through `launch` (returns a cudaError_t as int) and counts it.  A `timed` launch is bracketed
+// by an event pair while timing is on (gofr_engine_kernel_time_ms).  Called with the engine lock held.
+template <typename Launch>
+static int run_launch(gofr_engine* e, const char* what, bool timed, cudaStream_t st, Launch&& launch) {
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    timed = timed && e->timing_on;
+    if (timed) {
+        fold_timing(e);
+        CUDA_TRY(cudaEventCreate(&ev0));
+        CUDA_TRY(cudaEventCreate(&ev1));
+        CUDA_TRY(cudaEventRecord(ev0, st));
+    }
+    const int rc = launch();
+    if (rc != 0) { set_last_error("%s kernel launch failed: %s", what, cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
+    if (timed) {
+        CUDA_TRY(cudaEventRecord(ev1, st));
+        e->timing.emplace_back(ev0, ev1);
+    }
+    e->launches++;
+    return GOFR_OK;
+}
+
+// Start of a frame-style call (gRPC, proto, request log), engine lock held.  An empty batch only gets out_off[0] = 0;
+// otherwise the look-back state grows to the batch's tiles and p receives the fields every frame kernel shares.
+template <typename Params>
+static int frame_prologue(gofr_engine* e, uint32_t n, uint8_t* d_out, uint64_t out_cap, uint32_t* d_out_off, cudaStream_t st,
+                          Params* p) {
+    memset(p, 0, sizeof *p);
+    if (n == 0) {
+        if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st));
+        return GOFR_OK;
+    }
+    p->n = n;
+    p->n_tiles = (n + kServeThreads - 1) / kServeThreads;
+    { int rc = grow_state(e, p->n_tiles); if (rc) return rc; }
+    { int rc = next_epoch(e, &p->epoch); if (rc) return rc; }
+    p->out = d_out; p->out_cap = out_cap; p->out_off = d_out_off;
+    p->tile_state = e->d_state; p->overflow = e->d_flag;
+    return GOFR_OK;
+}
+
 // one fused launch; `state`/`flag` are scratch owned by the caller of this helper
 static int launch_one(gofr_engine* e, const void* d_desc, const void* d_ids, const uint8_t* d_arena, uint32_t n,
                       const char* date29, uint8_t* d_out, uint64_t out_cap, uint32_t* d_off, uint32_t* d_meta,
@@ -337,23 +417,11 @@ static int launch_one(gofr_engine* e, const void* d_desc, const void* d_ids, con
     p.slot_bytes = slot_bytes;
     p.debug_flags = e->debug_flags;
     memcpy(p.date, date29, 29);
-    int grid = (int)std::min<uint32_t>((uint32_t)(wide ? e->wide_grid : e->grid), p.n_tiles);
-    if (!slot_bytes) grid = std::max(1, std::min(grid, e->grid / engines_on_device(e->device)));  // look-back: see engines_on_device
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (e->timing_on) {
-        fold_timing(e);
-        CUDA_TRY(cudaEventCreate(&ev0));
-        CUDA_TRY(cudaEventCreate(&ev1));
-        CUDA_TRY(cudaEventRecord(ev0, stream));
-    }
-    int rc = launch_serve(p, grid, wide ? e->w_smem_bytes : e->smem_bytes, stream, wide, e->has_values);
-    if (rc != 0) { set_last_error("serve kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    if (e->timing_on) {
-        CUDA_TRY(cudaEventRecord(ev1, stream));
-        e->timing.emplace_back(ev0, ev1);
-    }
-    e->launches++;
-    return GOFR_OK;
+    const int grid = slot_bytes ? (int)std::min<uint32_t>((uint32_t)(wide ? e->wide_grid : e->grid), p.n_tiles)
+                                : lookback_grid(e, e->grid, p.n_tiles);
+    return run_launch(e, "serve", true, stream, [&] {
+        return launch_serve(p, grid, wide ? e->w_smem_bytes : e->smem_bytes, stream, wide, e->has_values);
+    });
 }
 
 extern "C" {
@@ -369,24 +437,8 @@ int gofr_serve_device(gofr_engine* e, const gofr_req_desc* d_desc, const uint8_t
         if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st));
         return GOFR_OK;
     }
-    size_t tiles = (n + 63) / 64;  // enough for any tile size in use (serve: kServeT, gRPC / log: 128)
-    if (tiles > e->state_tiles) {
-        // grow the look-back scratch; stream-ordered w.r.t. earlier launches because cudaFree synchronises
-        cudaFree(e->d_state);
-        e->d_state = nullptr;
-        CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
-        CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
-        e->state_tiles = tiles;
-    }
-    if (e->hdr.bind_row_words) {
-        size_t need = (size_t)n * e->hdr.bind_row_words * 4;
-        if (need > e->bind_cap) {
-            cudaFree(e->d_bind);
-            e->d_bind = nullptr;
-            CUDA_TRY(cudaMalloc(&e->d_bind, need + need / 4 + 256));
-            e->bind_cap = need + need / 4;
-        }
-    }
+    { int rc = grow_state(e, (n + 63) / 64); if (rc) return rc; }  // enough for any tile size in use (serve: kServeT, gRPC / log: 128)
+    { int rc = grow_bind(e, n); if (rc) return rc; }
     return launch_one(e, d_desc, d_trace_ids, d_arena, n, date29, d_out, out_cap, d_out_off, d_meta, e->d_state, e->d_flag,
                       e->d_bind, st);
 }
@@ -402,15 +454,7 @@ int gofr_serve_device_slots(gofr_engine* e, const gofr_req_desc* d_desc, const u
     if (n == 0) return GOFR_OK;
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
-    if (e->hdr.bind_row_words) {
-        size_t need = (size_t)n * e->hdr.bind_row_words * 4;
-        if (need > e->bind_cap) {
-            cudaFree(e->d_bind);
-            e->d_bind = nullptr;
-            CUDA_TRY(cudaMalloc(&e->d_bind, need + need / 4 + 256));
-            e->bind_cap = need + need / 4;
-        }
-    }
+    { int rc = grow_bind(e, n); if (rc) return rc; }
     // no look-back scratch: slots make the tiles independent of each other
     return launch_one(e, d_desc, d_trace_ids, d_arena, n, date29, d_out, (uint64_t)n * slot_bytes, d_out_len, d_meta, nullptr,
                       e->d_flag, e->d_bind, (cudaStream_t)stream, nullptr, slot_bytes);
@@ -494,20 +538,26 @@ static int grow(void** p, size_t* cap, size_t need, size_t slack) {
 // (include/gofr_b200.h states the same for device-resident callers), so a staging arena is never sized to the byte.
 static constexpr size_t kArenaSlack = 16;
 
-// A chunk = contiguous request range [lo, hi) and the arena byte range it covers.
-struct ChunkPlan { uint32_t lo, hi; uint32_t arena_lo, arena_hi; };
+// A chunk = contiguous request range [lo, hi) and the arena byte range [arena_lo, arena_hi) (16-byte granular) it covers.
+struct ChunkPlan {
+    uint32_t lo, hi;
+    uint32_t arena_lo, arena_hi;
+    size_t abytes() const { return (size_t)arena_hi - arena_lo; }
+};
 
-// The arena byte range [*alo, *ahi) (16-byte granular) that requests [lo, hi) reference.  All arithmetic in 64 bits: a
+// Chunk ci of a host batch (e->chunk requests each) and the arena bytes its requests reference: up to the end of each
+// request's data, or with path_only up to the end of its path (routing reads nothing else).  All arithmetic in 64 bits: a
 // descriptor with a huge arena_off or data_len (say a data_len taken from a Content-Length header) must be refused, not
 // wrap around and pass.
-static int chunk_arena_range(const gofr_req_batch* in, uint32_t lo, uint32_t hi, uint32_t* alo_out, uint32_t* ahi_out) {
+static int chunk_arena_range(const gofr_engine* e, const gofr_req_batch* in, size_t ci, bool path_only, ChunkPlan* c) {
+    const uint32_t lo = (uint32_t)(ci * e->chunk), hi = (uint32_t)std::min<uint64_t>(in->n, (uint64_t)lo + e->chunk);
     uint64_t alo = ~0ull, ahi = 0;
     const gofr_req_desc* dd = in->desc;
     for (uint32_t i = lo; i < hi; i++) {
         const uint64_t a = dd[i].arena_off;
-        const uint64_t dend = ((a + dd[i].path_len + dd[i].query_len + 3u) & ~3ull) + dd[i].data_len;
+        const uint64_t end = path_only ? a + dd[i].path_len : ((a + dd[i].path_len + dd[i].query_len + 3u) & ~3ull) + dd[i].data_len;
         alo = a < alo ? a : alo;
-        ahi = dend > ahi ? dend : ahi;
+        ahi = end > ahi ? end : ahi;
     }
     if (hi <= lo) alo = 0;
     alo &= ~15ull;
@@ -517,8 +567,51 @@ static int chunk_arena_range(const gofr_req_batch* in, uint32_t lo, uint32_t hi,
         return GOFR_ERR_INVALID;
     }
     if (ahi > alo && !in->arena) { set_last_error("requests reference arena bytes but the batch has no arena"); return GOFR_ERR_INVALID; }
-    *alo_out = (uint32_t)alo;
-    *ahi_out = (uint32_t)(ahi > alo ? ahi : alo);
+    *c = {lo, hi, (uint32_t)alo, (uint32_t)(ahi > alo ? ahi : alo)};
+    return GOFR_OK;
+}
+
+// Copies the chunk's arena bytes to dst.  The range is rounded out to 16 bytes, so its end may lie past the caller's arena.
+static int stage_arena(const gofr_req_batch* in, const ChunkPlan& c, uint8_t* dst, cudaStream_t st) {
+    if (!c.abytes()) return GOFR_OK;
+    const size_t avail = in->arena_bytes > c.arena_lo ? (size_t)in->arena_bytes - c.arena_lo : 0;
+    CUDA_TRY(cudaMemcpyAsync(dst, in->arena + c.arena_lo, std::min(c.abytes(), avail), cudaMemcpyHostToDevice, st));
+    return GOFR_OK;
+}
+
+// Device output buffer of a packed chunk: the fixed part of every response plus what its data bytes can expand to.
+static size_t packed_out_cap(const gofr_engine* e, uint32_t cn, size_t abytes) {
+    return std::min<size_t>((size_t)cn * (e->hdr.max_fixed_len + 64) + (size_t)image_data_expand(e->hdr) * abytes + 4096, 0xFFFFFFF0ull);
+}
+
+// Grows slot s for a chunk of cn requests, abytes of arena and obytes of output.  No earlier chunk may still use its
+// buffers (wait_slot_egress, or a synchronised slot stream).
+static int reserve_slot(gofr_engine* e, Slot& s, uint32_t cn, size_t abytes, size_t obytes) {
+    if (cn > s.cap_n) {
+        cudaFree(s.d_desc); cudaFree(s.d_ids); cudaFree(s.d_off); cudaFree(s.d_meta); cudaFree(s.d_state); cudaFree(s.d_bind);
+        s.d_desc = s.d_ids = nullptr; s.d_off = s.d_meta = nullptr; s.d_state = nullptr; s.d_bind = nullptr;
+        s.cap_n = 0;
+        const size_t c = (size_t)cn + cn / 4 + 256, tiles = (c + 63) / 64;
+        if (cudaMalloc(&s.d_desc, c * 16) != cudaSuccess || cudaMalloc(&s.d_ids, c * 16) != cudaSuccess ||
+            cudaMalloc(&s.d_off, (c + 1) * 4) != cudaSuccess || cudaMalloc(&s.d_meta, c * 4) != cudaSuccess ||
+            cudaMalloc(&s.d_state, tiles * 8) != cudaSuccess) { set_last_error("cudaMalloc failed for a %zu-request chunk", c); return GOFR_ERR_NOMEM; }
+        if (cudaMemset(s.d_state, 0, tiles * 8) != cudaSuccess) return GOFR_ERR_CUDA;
+        if (e->hdr.bind_row_words && cudaMalloc(&s.d_bind, c * e->hdr.bind_row_words * 4 + 256) != cudaSuccess) { set_last_error("cudaMalloc failed for Bind scratch"); return GOFR_ERR_NOMEM; }
+        s.cap_n = c;
+    }
+    if (!s.d_flag) { if (cudaMalloc(&s.d_flag, 64) != cudaSuccess || cudaMemset(s.d_flag, 0, 64) != cudaSuccess) return GOFR_ERR_NOMEM; }
+    int rc;
+    if ((rc = grow((void**)&s.d_arena, &s.cap_arena, abytes + kArenaSlack, 256))) return rc;
+    return grow((void**)&s.d_out, &s.cap_out, obytes, 256);
+}
+
+// The slot's previous chunk must have left before its buffers are overwritten: a wait on the copy stream, unless the
+// buffers have to grow (cudaFree needs the host to be sure).
+static int wait_slot_egress(gofr_engine* e, Slot& s, uint32_t cn, size_t abytes, size_t obytes) {
+    if (!s.egress_pending) return GOFR_OK;
+    if (cn > s.cap_n || abytes + kArenaSlack > s.cap_arena || obytes > s.cap_out) CUDA_TRY(cudaEventSynchronize(s.ev_egress));
+    else CUDA_TRY(cudaStreamWaitEvent(e->st_h2d, s.ev_egress, 0));
+    s.egress_pending = false;
     return GOFR_OK;
 }
 
@@ -569,90 +662,50 @@ static int batch_submit_locked(gofr_engine* e, const gofr_req_batch* in, gofr_re
     }
 
     // Chunks are contiguous request ranges; a chunk's arena range is the min/max over its descriptors.  The scan is done
-    // lazily, right before a chunk is enqueued, so it overlaps with the GPU work of the chunks already in flight
-    // (scanning all descriptors up front costs milliseconds of pure latency on a 1 Mi-request batch).
-    const size_t nchunks_total = n ? (n + e->chunk - 1) / e->chunk : 0;
-    std::vector<ChunkPlan> plan(nchunks_total);
-    std::vector<char> planned(nchunks_total, 0);
-    auto plan_chunk = [&](size_t ci) -> int {
-        if (planned[ci]) return GOFR_OK;
-        uint32_t lo = (uint32_t)(ci * e->chunk), hi = std::min<uint32_t>(n, lo + e->chunk);
-        uint32_t alo = 0, ahi = 0;
-        int prc = chunk_arena_range(in, lo, hi, &alo, &ahi);
-        if (prc) return prc;
-        plan[ci] = {lo, hi, alo, ahi};
-        planned[ci] = 1;
-        return GOFR_OK;
-    };
+    // right before a chunk is enqueued, so it overlaps with the GPU work of the chunks already in flight (scanning all
+    // descriptors up front costs milliseconds of pure latency on a 1 Mi-request batch).
+    const size_t nchunks = ((size_t)n + e->chunk - 1) / e->chunk;
     // ---- streaming path: caller buffers are pinned → egress is device driven, the host never blocks mid-batch ----
     auto device_visible = [](const void* p) {
         cudaPointerAttributes a;
         if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
         return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
     };
-    if (n && !getenv("GOFR_LEGACY_EGRESS") && device_visible(out->out) && device_visible(out->out_off) && device_visible(out->meta)) {
-        auto ensure_s = [&](Slot& s, uint32_t cn, size_t abytes, size_t ocap) -> int {
-            if (cn > s.cap_n) {
-                cudaFree(s.d_desc); cudaFree(s.d_ids); cudaFree(s.d_off); cudaFree(s.d_meta); cudaFree(s.d_state); cudaFree(s.d_bind);
-                s.d_desc = s.d_ids = nullptr; s.d_off = s.d_meta = nullptr; s.d_state = nullptr; s.d_bind = nullptr;
-                size_t c = (size_t)cn + cn / 4 + 256;
-                size_t tiles = (c + 63) / 64;
-                if (cudaMalloc(&s.d_desc, c * 16) != cudaSuccess || cudaMalloc(&s.d_ids, c * 16) != cudaSuccess ||
-                    cudaMalloc(&s.d_off, (c + 1) * 4) != cudaSuccess || cudaMalloc(&s.d_meta, c * 4) != cudaSuccess ||
-                    cudaMalloc(&s.d_state, tiles * 8) != cudaSuccess) { set_last_error("cudaMalloc failed for a %zu-request chunk", c); s.cap_n = 0; return GOFR_ERR_NOMEM; }
-                if (cudaMemset(s.d_state, 0, tiles * 8) != cudaSuccess) return GOFR_ERR_CUDA;
-                if (e->hdr.bind_row_words && cudaMalloc(&s.d_bind, c * e->hdr.bind_row_words * 4 + 256) != cudaSuccess) { s.cap_n = 0; return GOFR_ERR_NOMEM; }
-                s.cap_n = c;
-            }
-            if (!s.d_flag) { if (cudaMalloc(&s.d_flag, 64) != cudaSuccess || cudaMemset(s.d_flag, 0, 64) != cudaSuccess) return GOFR_ERR_NOMEM; }
-            int rc;
-            if ((rc = grow((void**)&s.d_arena, &s.cap_arena, abytes + kArenaSlack, 256))) return rc;
-            if ((rc = grow((void**)&s.d_out, &s.cap_out, ocap, 256))) return rc;
-            return GOFR_OK;
-        };
+    if (device_visible(out->out) && device_visible(out->out_off) && device_visible(out->meta)) {
         // growing buffers frees memory: make sure nothing from an earlier batch is still using them
         CUDA_TRY(cudaMemsetAsync(e->d_chain, 0, 8, e->st_compute));
         e->h_status[0] = 0; e->h_status[1] = 0;
-        for (size_t ci = 0; ci < plan.size(); ci++) {
+        for (size_t ci = 0; ci < nchunks; ci++) {
             Slot& s = e->slots[ci % kSlots];
-            { int prc = plan_chunk(ci); if (prc) return prc; }
-            const ChunkPlan& c = plan[ci];
-            uint32_t cn = c.hi - c.lo;
-            size_t abytes = (size_t)c.arena_hi - c.arena_lo;
-            size_t ocap = std::min<size_t>((size_t)cn * (e->hdr.max_fixed_len + 64) + (size_t)image_data_expand(e->hdr) * abytes + 4096, 0xFFFFFFF0ull);
-            if (s.egress_pending) {
-                // the slot's previous chunk must have left before its buffers are overwritten: a stream-side wait,
-                // unless the buffers have to grow (cudaFree needs the host to be sure)
-                const bool grows = cn > s.cap_n || abytes + kArenaSlack > s.cap_arena || ocap > s.cap_out;
-                if (grows) CUDA_TRY(cudaEventSynchronize(s.ev_egress));
-                else CUDA_TRY(cudaStreamWaitEvent(e->st_h2d, s.ev_egress, 0));
-                s.egress_pending = false;
-            }
-            int rc = ensure_s(s, cn, abytes, ocap);
+            ChunkInfo* info = e->d_info + ci % kSlots;
+            ChunkPlan c;
+            int rc = chunk_arena_range(e, in, ci, false, &c);
             if (rc) return rc;
+            const uint32_t cn = c.hi - c.lo;
+            const size_t ocap = packed_out_cap(e, cn, c.abytes());
+            if ((rc = wait_slot_egress(e, s, cn, c.abytes(), ocap))) return rc;
+            if ((rc = reserve_slot(e, s, cn, c.abytes(), ocap))) return rc;
             CUDA_TRY(cudaMemcpyAsync(s.d_desc, in->desc + c.lo, (size_t)cn * 16, cudaMemcpyHostToDevice, e->st_h2d));
             CUDA_TRY(cudaMemcpyAsync(s.d_ids, in->trace_ids + (size_t)c.lo * 16, (size_t)cn * 16, cudaMemcpyHostToDevice, e->st_h2d));
-            if (abytes) {
-                size_t avail = in->arena_bytes > c.arena_lo ? (size_t)in->arena_bytes - c.arena_lo : 0;
-                CUDA_TRY(cudaMemcpyAsync(s.d_arena, in->arena + c.arena_lo, std::min(abytes, avail), cudaMemcpyHostToDevice, e->st_h2d));
-            }
+            if ((rc = stage_arena(in, c, s.d_arena, e->st_h2d))) return rc;
             CUDA_TRY(cudaEventRecord(s.ev_h2d, e->st_h2d));
             CUDA_TRY(cudaStreamWaitEvent(e->st_compute, s.ev_h2d, 0));
             rc = launch_one(e, s.d_desc, s.d_ids, s.d_arena - c.arena_lo, cn, in->date, s.d_out, s.cap_out, s.d_off, s.d_meta,
                             s.d_state, s.d_flag, s.d_bind, e->st_compute, e->d_chain);
             if (rc) return rc;
-            if (launch_advance(e->d_chain, s.d_off, cn, s.d_flag, e->d_info + (ci % kSlots), out->out_cap, e->st_compute) != 0) {
-                set_last_error("advance kernel launch failed"); return GOFR_ERR_CUDA;
-            }
+            rc = run_launch(e, "advance", false, e->st_compute, [&] {
+                return launch_advance(e->d_chain, s.d_off, cn, s.d_flag, info, out->out_cap, e->st_compute);
+            });
+            if (rc) return rc;
             CUDA_TRY(cudaEventRecord(s.ev_served, e->st_compute));
             CUDA_TRY(cudaStreamWaitEvent(e->st_egress, s.ev_served, 0));
-            if (launch_egress(e->d_info + (ci % kSlots), s.d_out, s.d_off, s.d_meta, cn, out->out, out->out_off + c.lo,
-                              out->meta + c.lo, e->h_status, e->egress_grid, e->st_egress) != 0) {
-                set_last_error("egress kernel launch failed"); return GOFR_ERR_CUDA;
-            }
+            rc = run_launch(e, "egress", false, e->st_egress, [&] {
+                return launch_egress(info, s.d_out, s.d_off, s.d_meta, cn, out->out, out->out_off + c.lo, out->meta + c.lo,
+                                     e->h_status, e->egress_grid, e->st_egress);
+            });
+            if (rc) return rc;
             CUDA_TRY(cudaEventRecord(s.ev_egress, e->st_egress));
             s.egress_pending = true;
-            e->launches += 2;
         }
         CUDA_TRY(cudaMemcpyAsync((void*)&e->h_status[0], e->d_chain, 8, cudaMemcpyDeviceToHost, e->st_egress));
         CUDA_TRY(wait_batch(e, n));
@@ -667,48 +720,22 @@ static int batch_submit_locked(gofr_engine* e, const gofr_req_batch* in, gofr_re
     }
 
     // ---- straightforward 3-slot software pipeline ----
-    auto ensure = [&](Slot& s, uint32_t cn, size_t abytes, size_t ocap) -> int {
-        int rc;
-        if (cn > s.cap_n) {
-            cudaFree(s.d_desc); cudaFree(s.d_ids); cudaFree(s.d_off); cudaFree(s.d_meta); cudaFree(s.d_state); cudaFree(s.d_bind);
-            s.d_desc = s.d_ids = nullptr; s.d_off = s.d_meta = nullptr; s.d_state = nullptr; s.d_bind = nullptr;
-            size_t c = (size_t)cn + cn / 4 + 256;
-            size_t tiles = (c + 63) / 64;
-            if (cudaMalloc(&s.d_desc, c * 16) != cudaSuccess || cudaMalloc(&s.d_ids, c * 16) != cudaSuccess ||
-                cudaMalloc(&s.d_off, (c + 1) * 4) != cudaSuccess || cudaMalloc(&s.d_meta, c * 4) != cudaSuccess ||
-                cudaMalloc(&s.d_state, tiles * 8) != cudaSuccess) { set_last_error("cudaMalloc failed for a %zu-request chunk", c); s.cap_n = 0; return GOFR_ERR_NOMEM; }
-            if (cudaMemset(s.d_state, 0, tiles * 8) != cudaSuccess) return GOFR_ERR_CUDA;
-            if (e->hdr.bind_row_words && cudaMalloc(&s.d_bind, c * e->hdr.bind_row_words * 4 + 256) != cudaSuccess) { set_last_error("cudaMalloc failed for Bind scratch"); s.cap_n = 0; return GOFR_ERR_NOMEM; }
-            s.cap_n = c;
-        }
-        if (!s.d_flag) { if (cudaMalloc(&s.d_flag, 64) != cudaSuccess || cudaMemset(s.d_flag, 0, 64) != cudaSuccess) return GOFR_ERR_NOMEM; }
-        if ((rc = grow((void**)&s.d_arena, &s.cap_arena, abytes + kArenaSlack, 256))) return rc;
-        if ((rc = grow((void**)&s.d_out, &s.cap_out, ocap, 256))) return rc;
-        return GOFR_OK;
-    };
-
+    ChunkPlan plan[kSlots];  // the chunk each slot holds
     size_t issued = 0, finished = 0;
     uint64_t write_pos = 0;
-    const size_t nchunks = plan.size();
     // issue order == completion order == chunk order; out offsets are rebased on the host as chunks complete
     while (finished < nchunks) {
         // keep up to kSlots chunks in flight
         while (issued < nchunks && issued - finished < (size_t)kSlots) {
-            int si = (int)(issued % kSlots);
-            Slot& s = e->slots[si];
-            { int prc = plan_chunk(issued); if (prc) return prc; }
-            const ChunkPlan& c = plan[issued];
-            uint32_t cn = c.hi - c.lo;
-            size_t abytes = (size_t)c.arena_hi - c.arena_lo;
-            size_t ocap = std::min<size_t>((size_t)cn * (e->hdr.max_fixed_len + 64) + (size_t)image_data_expand(e->hdr) * abytes + 4096, 0xFFFFFFF0ull);
-            int rc = ensure(s, cn, abytes, ocap);
+            Slot& s = e->slots[issued % kSlots];
+            ChunkPlan& c = plan[issued % kSlots];
+            int rc = chunk_arena_range(e, in, issued, false, &c);
             if (rc) return rc;
+            const uint32_t cn = c.hi - c.lo;
+            if ((rc = reserve_slot(e, s, cn, c.abytes(), packed_out_cap(e, cn, c.abytes())))) return rc;
             CUDA_TRY(cudaMemcpyAsync(s.d_desc, in->desc + c.lo, (size_t)cn * 16, cudaMemcpyHostToDevice, s.stream));
             CUDA_TRY(cudaMemcpyAsync(s.d_ids, in->trace_ids + (size_t)c.lo * 16, (size_t)cn * 16, cudaMemcpyHostToDevice, s.stream));
-            if (abytes) {
-                size_t avail = in->arena_bytes > c.arena_lo ? (size_t)in->arena_bytes - c.arena_lo : 0;
-                CUDA_TRY(cudaMemcpyAsync(s.d_arena, in->arena + c.arena_lo, std::min(abytes, avail), cudaMemcpyHostToDevice, s.stream));
-            }
+            if ((rc = stage_arena(in, c, s.d_arena, s.stream))) return rc;
             // descriptors keep absolute arena offsets: pass a rebased arena pointer
             rc = launch_one(e, s.d_desc, s.d_ids, s.d_arena - c.arena_lo, cn, in->date, s.d_out, s.cap_out, s.d_off, s.d_meta,
                             s.d_state, s.d_flag, s.d_bind, s.stream);
@@ -721,9 +748,8 @@ static int batch_submit_locked(gofr_engine* e, const gofr_req_batch* in, gofr_re
             issued++;
         }
         // retire the oldest chunk: learn its size, then pull exactly that many bytes
-        int si = (int)(finished % kSlots);
-        Slot& s = e->slots[si];
-        const ChunkPlan& c = plan[finished];
+        Slot& s = e->slots[finished % kSlots];
+        const ChunkPlan& c = plan[finished % kSlots];
         CUDA_TRY(cudaEventSynchronize(s.done));
         uint32_t total = s.h_tail[0];
         if (s.h_tail[1]) { CUDA_TRY(cudaMemsetAsync(s.d_flag, 0, 4, s.stream)); final_rc = GOFR_ERR_CAPACITY; set_last_error("device output buffer too small for chunk %zu", finished); total = 0; }
@@ -756,45 +782,24 @@ int gofr_batch_submit_slots(gofr_engine* e, const gofr_req_batch* in, gofr_slot_
 static int batch_submit_slots_locked(gofr_engine* e, const gofr_req_batch* in, gofr_slot_batch* out, gofr_ticket* ticket) {
     const uint32_t n = in->n, slot = out->slot_bytes;
     int final_rc = GOFR_OK;
-    const size_t nchunks = n ? (n + e->chunk - 1) / e->chunk : 0;
+    const size_t nchunks = ((size_t)n + e->chunk - 1) / e->chunk;
     for (size_t ci = 0; ci < nchunks; ci++) {
         Slot& s = e->slots[ci % kSlots];
         // the chunk's request range and the arena bytes it covers (scanned right before the chunk is enqueued)
-        const uint32_t lo = (uint32_t)(ci * e->chunk), hi = std::min<uint32_t>(n, lo + e->chunk), cn = hi - lo;
-        uint32_t alo = 0, ahi = 0;
-        { int prc = chunk_arena_range(in, lo, hi, &alo, &ahi); if (prc) return prc; }
-        const size_t abytes = (size_t)ahi - alo, obytes = (size_t)cn * slot;
-        if (s.egress_pending) {  // the slot's previous chunk must have left before its buffers are reused
-            const bool grows = cn > s.cap_n || abytes + kArenaSlack > s.cap_arena || obytes > s.cap_out;
-            if (grows) CUDA_TRY(cudaEventSynchronize(s.ev_egress));
-            else CUDA_TRY(cudaStreamWaitEvent(e->st_h2d, s.ev_egress, 0));
-            s.egress_pending = false;
-        }
-        if (cn > s.cap_n) {
-            cudaFree(s.d_desc); cudaFree(s.d_ids); cudaFree(s.d_off); cudaFree(s.d_meta); cudaFree(s.d_state); cudaFree(s.d_bind);
-            s.d_desc = s.d_ids = nullptr; s.d_off = s.d_meta = nullptr; s.d_state = nullptr; s.d_bind = nullptr;
-            const size_t c = (size_t)cn + cn / 4 + 256, tiles = (c + 63) / 64;
-            if (cudaMalloc(&s.d_desc, c * 16) != cudaSuccess || cudaMalloc(&s.d_ids, c * 16) != cudaSuccess ||
-                cudaMalloc(&s.d_off, (c + 1) * 4) != cudaSuccess || cudaMalloc(&s.d_meta, c * 4) != cudaSuccess ||
-                cudaMalloc(&s.d_state, tiles * 8) != cudaSuccess) { set_last_error("cudaMalloc failed for a %zu-request chunk", c); s.cap_n = 0; return GOFR_ERR_NOMEM; }
-            if (cudaMemset(s.d_state, 0, tiles * 8) != cudaSuccess) return GOFR_ERR_CUDA;
-            if (e->hdr.bind_row_words && cudaMalloc(&s.d_bind, c * e->hdr.bind_row_words * 4 + 256) != cudaSuccess) { s.cap_n = 0; return GOFR_ERR_NOMEM; }
-            s.cap_n = c;
-        }
-        if (!s.d_flag) { if (cudaMalloc(&s.d_flag, 64) != cudaSuccess || cudaMemset(s.d_flag, 0, 64) != cudaSuccess) return GOFR_ERR_NOMEM; }
-        int rc;
-        if ((rc = grow((void**)&s.d_arena, &s.cap_arena, abytes + kArenaSlack, 256))) return rc;
-        if ((rc = grow((void**)&s.d_out, &s.cap_out, obytes, 256))) return rc;
+        ChunkPlan c;
+        int rc = chunk_arena_range(e, in, ci, false, &c);
+        if (rc) return rc;
+        const uint32_t lo = c.lo, cn = c.hi - c.lo;
+        const size_t obytes = (size_t)cn * slot;
+        if ((rc = wait_slot_egress(e, s, cn, c.abytes(), obytes))) return rc;
+        if ((rc = reserve_slot(e, s, cn, c.abytes(), obytes))) return rc;
         CUDA_TRY(cudaMemcpyAsync(s.d_desc, in->desc + lo, (size_t)cn * 16, cudaMemcpyHostToDevice, e->st_h2d));
         CUDA_TRY(cudaMemcpyAsync(s.d_ids, in->trace_ids + (size_t)lo * 16, (size_t)cn * 16, cudaMemcpyHostToDevice, e->st_h2d));
-        if (abytes) {
-            const size_t avail = in->arena_bytes > alo ? (size_t)in->arena_bytes - alo : 0;
-            CUDA_TRY(cudaMemcpyAsync(s.d_arena, in->arena + alo, std::min(abytes, avail), cudaMemcpyHostToDevice, e->st_h2d));
-        }
+        if ((rc = stage_arena(in, c, s.d_arena, e->st_h2d))) return rc;
         CUDA_TRY(cudaEventRecord(s.ev_h2d, e->st_h2d));
         CUDA_TRY(cudaStreamWaitEvent(e->st_compute, s.ev_h2d, 0));
-        rc = launch_one(e, s.d_desc, s.d_ids, s.d_arena - alo, cn, in->date, s.d_out, obytes, s.d_off, s.d_meta, s.d_state, s.d_flag,
-                        s.d_bind, e->st_compute, nullptr, slot);
+        rc = launch_one(e, s.d_desc, s.d_ids, s.d_arena - c.arena_lo, cn, in->date, s.d_out, obytes, s.d_off, s.d_meta, s.d_state,
+                        s.d_flag, s.d_bind, e->st_compute, nullptr, slot);
         if (rc) return rc;
         CUDA_TRY(cudaEventRecord(s.ev_served, e->st_compute));
         CUDA_TRY(cudaStreamWaitEvent(e->st_egress, s.ev_served, 0));
@@ -909,37 +914,12 @@ int gofr_grpc_hello_device(gofr_engine* e, const uint8_t* d_in, const uint32_t* 
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (n == 0) { if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st)); return GOFR_OK; }
-    size_t tiles = (n + kServeThreads - 1) / kServeThreads;
-    if (tiles > e->state_tiles) {
-        cudaFree(e->d_state);
-        e->d_state = nullptr;
-        CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
-        CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
-        e->state_tiles = tiles;
-    }
-    if (e->grpc_grid <= 0) {
-        e->grpc_grid = grpc_max_grid(e->device);
-        if (e->grpc_grid <= 0) { set_last_error("grpc kernel cannot be resident"); return GOFR_ERR_CUDA; }
-    }
     GrpcParams p;
-    memset(&p, 0, sizeof p);
-    p.in = d_in; p.in_off = d_in_off; p.n = n; p.n_tiles = (uint32_t)tiles;
-    { int erc = next_epoch(e, &p.epoch); if (erc) return erc; }
-    p.out = d_out; p.out_cap = out_cap; p.out_off = d_out_off; p.meta = d_meta;
-    p.tile_state = e->d_state; p.overflow = e->d_flag;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (e->timing_on) {
-        fold_timing(e);
-        CUDA_TRY(cudaEventCreate(&ev0));
-        CUDA_TRY(cudaEventCreate(&ev1));
-        CUDA_TRY(cudaEventRecord(ev0, st));
-    }
-    int rc = launch_grpc_hello(p, (int)std::min<size_t>((size_t)std::max(1, e->grpc_grid / engines_on_device(e->device)), tiles), st);
-    if (rc != 0) { set_last_error("grpc kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    if (e->timing_on) { CUDA_TRY(cudaEventRecord(ev1, st)); e->timing.emplace_back(ev0, ev1); }
-    e->launches++;
-    return GOFR_OK;
+    { int rc = frame_prologue(e, n, d_out, out_cap, d_out_off, st, &p); if (rc || n == 0) return rc; }
+    { int rc = lazy_grid(e, &e->grpc_grid, grpc_max_grid, "grpc"); if (rc) return rc; }
+    p.in = d_in; p.in_off = d_in_off; p.meta = d_meta;
+    const int grid = lookback_grid(e, e->grpc_grid, p.n_tiles);
+    return run_launch(e, "grpc", true, st, [&] { return launch_grpc_hello(p, grid, st); });
 }
 
 // rows → frames (decode == false) or frames → rows (decode == true): the same launch plumbing, two codecs
@@ -967,39 +947,13 @@ static int proto_run(gofr_engine* e, const gofr_proto_field* fields, uint32_t n_
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (n == 0) { if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st)); return GOFR_OK; }
-    size_t tiles = (n + kServeThreads - 1) / kServeThreads;
-    if (tiles > e->state_tiles) {
-        cudaFree(e->d_state);
-        e->d_state = nullptr;
-        CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
-        CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
-        e->state_tiles = tiles;
-    }
-    int& grid = decode ? e->proto_decode_grid : e->proto_grid;
-    if (grid <= 0) {
-        grid = decode ? proto_decode_max_grid(e->device) : proto_max_grid(e->device);
-        if (grid <= 0) { set_last_error("proto kernel cannot be resident"); return GOFR_ERR_CUDA; }
-    }
     GrpcParams p;
-    memset(&p, 0, sizeof p);
-    p.in = d_rows; p.in_off = d_row_off; p.n = n; p.n_tiles = (uint32_t)tiles;
-    { int erc = next_epoch(e, &p.epoch); if (erc) return erc; }
-    p.out = d_out; p.out_cap = out_cap; p.out_off = d_out_off; p.meta = d_meta;
-    p.tile_state = e->d_state; p.overflow = e->d_flag;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (e->timing_on) {
-        fold_timing(e);
-        CUDA_TRY(cudaEventCreate(&ev0));
-        CUDA_TRY(cudaEventCreate(&ev1));
-        CUDA_TRY(cudaEventRecord(ev0, st));
-    }
-    const int g_ = (int)std::min<size_t>((size_t)std::max(1, grid / engines_on_device(e->device)), tiles);
-    int rc = decode ? launch_proto_decode(p, S, g_, st) : launch_proto_encode(p, S, g_, st);
-    if (rc != 0) { set_last_error("proto kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    if (e->timing_on) { CUDA_TRY(cudaEventRecord(ev1, st)); e->timing.emplace_back(ev0, ev1); }
-    e->launches++;
-    return GOFR_OK;
+    { int rc = frame_prologue(e, n, d_out, out_cap, d_out_off, st, &p); if (rc || n == 0) return rc; }
+    int& grid = decode ? e->proto_decode_grid : e->proto_grid;
+    { int rc = lazy_grid(e, &grid, decode ? proto_decode_max_grid : proto_max_grid, "proto"); if (rc) return rc; }
+    p.in = d_rows; p.in_off = d_row_off; p.meta = d_meta;
+    const int g_ = lookback_grid(e, grid, p.n_tiles);
+    return run_launch(e, "proto", true, st, [&] { return decode ? launch_proto_decode(p, S, g_, st) : launch_proto_encode(p, S, g_, st); });
 }
 
 // message types with nested / repeated fields -> the kernel's descriptor: validation, words of every fixed part, nesting depth
@@ -1074,31 +1028,13 @@ static int proto_nested_run(gofr_engine* e, const gofr_proto_nmsg* msgs, uint32_
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (n == 0) { if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st)); return GOFR_OK; }
-    size_t tiles = (n + kServeThreads - 1) / kServeThreads;
-    if (tiles > e->state_tiles) {
-        cudaFree(e->d_state);
-        e->d_state = nullptr;
-        CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
-        CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
-        e->state_tiles = tiles;
-    }
-    int& grid = decode ? e->proto_nested_decode_grid : e->proto_nested_grid;
-    if (grid <= 0) {
-        grid = decode ? proto_nested_decode_max_grid(e->device) : proto_nested_max_grid(e->device);
-        if (grid <= 0) { set_last_error("proto kernel cannot be resident"); return GOFR_ERR_CUDA; }
-    }
     GrpcParams p;
-    memset(&p, 0, sizeof p);
-    p.in = d_in; p.in_off = d_in_off; p.n = n; p.n_tiles = (uint32_t)tiles;
-    { int erc = next_epoch(e, &p.epoch); if (erc) return erc; }
-    p.out = d_out; p.out_cap = out_cap; p.out_off = d_out_off; p.meta = d_meta;
-    p.tile_state = e->d_state; p.overflow = e->d_flag;
-    const int g_ = (int)std::min<size_t>((size_t)std::max(1, grid / engines_on_device(e->device)), tiles);
-    int rc = decode ? launch_proto_decode_nested(p, D, g_, st) : launch_proto_encode_nested(p, D, g_, st);
-    if (rc != 0) { set_last_error("proto kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    e->launches++;
-    return GOFR_OK;
+    { int rc = frame_prologue(e, n, d_out, out_cap, d_out_off, st, &p); if (rc || n == 0) return rc; }
+    int& grid = decode ? e->proto_nested_decode_grid : e->proto_nested_grid;
+    { int rc = lazy_grid(e, &grid, decode ? proto_nested_decode_max_grid : proto_nested_max_grid, "proto"); if (rc) return rc; }
+    p.in = d_in; p.in_off = d_in_off; p.meta = d_meta;
+    const int g_ = lookback_grid(e, grid, p.n_tiles);
+    return run_launch(e, "proto", false, st, [&] { return decode ? launch_proto_decode_nested(p, D, g_, st) : launch_proto_encode_nested(p, D, g_, st); });
 }
 
 int gofr_proto_encode_nested_device(gofr_engine* e, const gofr_proto_nmsg* msgs, uint32_t n_msgs, const gofr_proto_nfield* fields,
@@ -1146,9 +1082,15 @@ int gofr_route_device(gofr_engine* e, const gofr_req_desc* d_desc, const uint8_t
     memset(&p, 0, sizeof p);
     p.desc = d_desc; p.arena = d_arena; p.n = n; p.image = e->d_image; p.hot_bytes = e->hdr.hot_bytes;
     p.meta = d_meta; p.vars = d_vars;
-    int rc = launch_route(p, e->sm_count, stream);
-    if (rc != 0) { set_last_error("route kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    e->launches++;
+    return run_launch(e, "route", false, (cudaStream_t)stream, [&] { return launch_route(p, e->sm_count, stream); });
+}
+
+// The table index of schema_id, which must be a schema Bind can fill.
+static int bindable_schema(const gofr_engine* e, uint32_t schema_id, uint32_t* sidx) {
+    *sidx = 0xFFFFFFFFu;
+    for (size_t k = 0; k < e->schema_ids.size(); k++) if (e->schema_ids[k] == schema_id) *sidx = (uint32_t)k;
+    if (*sidx == 0xFFFFFFFFu) { set_last_error("schema %u is not part of the engine's table", schema_id); return GOFR_ERR_INVALID; }
+    if (!(e->schema_flags[*sidx] & SF_BINDABLE)) { set_last_error("schema %u: Bind takes flat structs of int / float64 / bool / string fields only", schema_id); return GOFR_ERR_UNSUPPORTED; }
     return GOFR_OK;
 }
 
@@ -1156,10 +1098,8 @@ int gofr_bind_device(gofr_engine* e, uint32_t schema_id, const gofr_req_desc* d_
                      uint8_t* d_rows, uint32_t slot_bytes, uint32_t* d_len, uint32_t* d_status, void* stream) {
     if (!e || (n && (!d_desc || !d_arena || !d_rows || !d_len || !d_status))) return GOFR_ERR_INVALID;
     if (slot_bytes == 0 || (slot_bytes & 15u) || ((uintptr_t)d_rows & 15u)) { set_last_error("slot_bytes must be a positive multiple of 16 and d_rows 16-byte aligned"); return GOFR_ERR_INVALID; }
-    uint32_t sidx = 0xFFFFFFFFu;
-    for (size_t k = 0; k < e->schema_ids.size(); k++) if (e->schema_ids[k] == schema_id) sidx = (uint32_t)k;
-    if (sidx == 0xFFFFFFFFu) { set_last_error("schema %u is not part of the engine's table", schema_id); return GOFR_ERR_INVALID; }
-    if (!(e->schema_flags[sidx] & SF_BINDABLE)) { set_last_error("schema %u: Bind takes flat structs of int / float64 / bool / string fields only", schema_id); return GOFR_ERR_UNSUPPORTED; }
+    uint32_t sidx = 0;
+    { int rc = bindable_schema(e, schema_id, &sidx); if (rc) return rc; }
     if (n == 0) return GOFR_OK;
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
@@ -1167,47 +1107,35 @@ int gofr_bind_device(gofr_engine* e, uint32_t schema_id, const gofr_req_desc* d_
     memset(&p, 0, sizeof p);
     p.desc = d_desc; p.arena = d_arena; p.n = n; p.image = e->d_image; p.hot_bytes = e->hdr.hot_bytes; p.schema_idx = sidx;
     p.out = d_rows; p.slot_bytes = slot_bytes; p.len = d_len; p.status = d_status;
-    int rc = launch_bind(p, e->sm_count, stream);
-    if (rc != 0) { set_last_error("bind kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    e->launches++;
-    return GOFR_OK;
+    return run_launch(e, "bind", false, (cudaStream_t)stream, [&] { return launch_bind(p, e->sm_count, stream); });
 }
 
 int gofr_batch_bind(gofr_engine* e, uint32_t schema_id, const gofr_req_batch* in, uint8_t* rows, uint32_t slot_bytes,
                     uint32_t* len, uint32_t* status) {
     if (!e || !in || (in->n && (!in->desc || !rows || !len || !status))) return GOFR_ERR_INVALID;
     if (slot_bytes == 0 || (slot_bytes & 15u)) { set_last_error("slot_bytes must be a positive multiple of 16"); return GOFR_ERR_INVALID; }
-    uint32_t sidx = 0xFFFFFFFFu;
-    for (size_t k = 0; k < e->schema_ids.size(); k++) if (e->schema_ids[k] == schema_id) sidx = (uint32_t)k;
-    if (sidx == 0xFFFFFFFFu) { set_last_error("schema %u is not part of the engine's table", schema_id); return GOFR_ERR_INVALID; }
-    if (!(e->schema_flags[sidx] & SF_BINDABLE)) { set_last_error("schema %u: Bind takes flat structs of int / float64 / bool / string fields only", schema_id); return GOFR_ERR_UNSUPPORTED; }
+    uint32_t sidx = 0;
+    { int rc = bindable_schema(e, schema_id, &sidx); if (rc) return rc; }
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
-    const uint32_t n = in->n;
-    for (uint32_t lo = 0; lo < n; lo += e->chunk) {
-        const uint32_t hi = std::min<uint32_t>(n, lo + e->chunk), cn = hi - lo;
-        uint32_t alo = 0, ahi = 0;
-        { int prc = chunk_arena_range(in, lo, hi, &alo, &ahi); if (prc) return prc; }
-        const size_t abytes = (size_t)ahi - alo;
-        int rc;
+    for (size_t ci = 0; ci * e->chunk < in->n; ci++) {
+        ChunkPlan c;
+        int rc = chunk_arena_range(e, in, ci, false, &c);
+        if (rc) return rc;
+        const uint32_t lo = c.lo, cn = c.hi - c.lo;
         if ((rc = grow((void**)&e->d_rt_desc, &e->rt_desc_cap, (size_t)cn * 16, 256))) return rc;
-        if ((rc = grow((void**)&e->d_rt_arena, &e->rt_arena_cap, abytes + 16, 256))) return rc;
+        if ((rc = grow((void**)&e->d_rt_arena, &e->rt_arena_cap, c.abytes() + kArenaSlack, 256))) return rc;
         if ((rc = grow((void**)&e->d_rt_meta, &e->rt_meta_cap, (size_t)cn * 8, 256))) return rc;
         if ((rc = grow((void**)&e->d_rt_rows, &e->rt_rows_cap, (size_t)cn * slot_bytes, 256))) return rc;
         cudaStream_t st = e->st_compute;
         CUDA_TRY(cudaMemcpyAsync(e->d_rt_desc, in->desc + lo, (size_t)cn * 16, cudaMemcpyHostToDevice, st));
-        if (abytes) {
-            const size_t avail = in->arena_bytes > alo ? (size_t)in->arena_bytes - alo : 0;
-            CUDA_TRY(cudaMemcpyAsync(e->d_rt_arena, in->arena + alo, std::min(abytes, avail), cudaMemcpyHostToDevice, st));
-        }
+        if ((rc = stage_arena(in, c, e->d_rt_arena, st))) return rc;
         BindParams p;
         memset(&p, 0, sizeof p);
-        p.desc = e->d_rt_desc; p.arena = e->d_rt_arena - alo; p.n = cn; p.image = e->d_image; p.hot_bytes = e->hdr.hot_bytes;
+        p.desc = e->d_rt_desc; p.arena = e->d_rt_arena - c.arena_lo; p.n = cn; p.image = e->d_image; p.hot_bytes = e->hdr.hot_bytes;
         p.schema_idx = sidx; p.out = e->d_rt_rows; p.slot_bytes = slot_bytes;
         p.len = (uint32_t*)e->d_rt_meta; p.status = (uint32_t*)e->d_rt_meta + cn;
-        rc = launch_bind(p, e->sm_count, st);
-        if (rc != 0) { set_last_error("bind kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-        e->launches++;
+        if ((rc = run_launch(e, "bind", false, st, [&] { return launch_bind(p, e->sm_count, st); }))) return rc;
         CUDA_TRY(cudaMemcpyAsync(rows + (size_t)lo * slot_bytes, e->d_rt_rows, (size_t)cn * slot_bytes, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaMemcpyAsync(len + lo, p.len, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaMemcpyAsync(status + lo, p.status, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
@@ -1220,40 +1148,23 @@ int gofr_batch_route(gofr_engine* e, const gofr_req_batch* in, uint32_t* meta, u
     if (!e || !in || (in->n && (!in->desc || !meta || !vars))) return GOFR_ERR_INVALID;
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
-    const uint32_t n = in->n;
-    for (uint32_t lo = 0; lo < n; lo += e->chunk) {
-        const uint32_t hi = std::min<uint32_t>(n, lo + e->chunk), cn = hi - lo;
-        uint64_t alo64 = ~0ull, ahi64 = 0;
-        for (uint32_t i = lo; i < hi; i++) {  // routing reads the path only
-            const gofr_req_desc& d = in->desc[i];
-            const uint64_t a = d.arena_off, b = a + d.path_len;
-            alo64 = a < alo64 ? a : alo64;
-            ahi64 = b > ahi64 ? b : ahi64;
-        }
-        alo64 &= ~15ull;
-        ahi64 = (ahi64 + 15ull) & ~15ull;
-        if (ahi64 > (((uint64_t)in->arena_bytes + 15ull) & ~15ull) || ahi64 > 0xFFFFFFF0ull) { set_last_error("a descriptor of requests %u..%u points outside the arena", lo, hi); return GOFR_ERR_INVALID; }
-        if (ahi64 > alo64 && !in->arena) { set_last_error("requests reference arena bytes but the batch has no arena"); return GOFR_ERR_INVALID; }
-        const uint32_t alo = (uint32_t)alo64, ahi = (uint32_t)(ahi64 > alo64 ? ahi64 : alo64);
-        const size_t abytes = (size_t)ahi - alo;
-        int rc;
+    for (size_t ci = 0; ci * e->chunk < in->n; ci++) {
+        ChunkPlan c;
+        int rc = chunk_arena_range(e, in, ci, true, &c);
+        if (rc) return rc;
+        const uint32_t lo = c.lo, cn = c.hi - c.lo;
         if ((rc = grow((void**)&e->d_rt_desc, &e->rt_desc_cap, (size_t)cn * 16, 256))) return rc;
-        if ((rc = grow((void**)&e->d_rt_arena, &e->rt_arena_cap, abytes + 16, 256))) return rc;
+        if ((rc = grow((void**)&e->d_rt_arena, &e->rt_arena_cap, c.abytes() + kArenaSlack, 256))) return rc;
         if ((rc = grow((void**)&e->d_rt_meta, &e->rt_meta_cap, (size_t)cn * 4, 256))) return rc;
         if ((rc = grow((void**)&e->d_rt_vars, &e->rt_vars_cap, (size_t)cn * 4 * GOFR_MAX_PATH_VARS, 256))) return rc;
         cudaStream_t st = e->st_compute;
         CUDA_TRY(cudaMemcpyAsync(e->d_rt_desc, in->desc + lo, (size_t)cn * 16, cudaMemcpyHostToDevice, st));
-        if (abytes) {
-            const size_t avail = in->arena_bytes > alo ? (size_t)in->arena_bytes - alo : 0;
-            CUDA_TRY(cudaMemcpyAsync(e->d_rt_arena, in->arena + alo, std::min(abytes, avail), cudaMemcpyHostToDevice, st));
-        }
+        if ((rc = stage_arena(in, c, e->d_rt_arena, st))) return rc;
         RouteParams p;
         memset(&p, 0, sizeof p);
-        p.desc = (const gofr_req_desc*)e->d_rt_desc; p.arena = e->d_rt_arena - alo; p.n = cn; p.image = e->d_image;
+        p.desc = (const gofr_req_desc*)e->d_rt_desc; p.arena = e->d_rt_arena - c.arena_lo; p.n = cn; p.image = e->d_image;
         p.hot_bytes = e->hdr.hot_bytes; p.meta = (uint32_t*)e->d_rt_meta; p.vars = (uint32_t*)e->d_rt_vars;
-        rc = launch_route(p, e->sm_count, st);
-        if (rc != 0) { set_last_error("route kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-        e->launches++;
+        if ((rc = run_launch(e, "route", false, st, [&] { return launch_route(p, e->sm_count, st); }))) return rc;
         CUDA_TRY(cudaMemcpyAsync(meta + lo, e->d_rt_meta, (size_t)cn * 4, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaMemcpyAsync(vars + (size_t)lo * GOFR_MAX_PATH_VARS, e->d_rt_vars, (size_t)cn * 4 * GOFR_MAX_PATH_VARS, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
@@ -1267,27 +1178,14 @@ int gofr_http_parse_device(gofr_engine* e, const uint8_t* d_raw, const uint32_t*
     if (n == 0) return GOFR_OK;
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
-    if (e->http_grid <= 0) {
-        e->http_grid = http_max_grid(e->device);
-        if (e->http_grid <= 0) { set_last_error("http kernel cannot be resident"); return GOFR_ERR_CUDA; }
-    }
+    { int rc = lazy_grid(e, &e->http_grid, http_max_grid, "http"); if (rc) return rc; }
     HttpParams p;
     memset(&p, 0, sizeof p);
     p.raw = d_raw; p.raw_off = d_raw_off; p.n = n; p.n_tiles = (n + kServeThreads - 1) / kServeThreads;
     p.desc = d_desc; p.arena = d_arena; p.status = d_status; p.spans = (unsigned long long*)d_spans;
     cudaStream_t st = (cudaStream_t)stream;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (e->timing_on) {
-        fold_timing(e);
-        CUDA_TRY(cudaEventCreate(&ev0));
-        CUDA_TRY(cudaEventCreate(&ev1));
-        CUDA_TRY(cudaEventRecord(ev0, st));
-    }
-    int rc = launch_http_parse(p, (int)std::min<uint32_t>((uint32_t)e->http_grid, p.n_tiles), st);
-    if (rc != 0) { set_last_error("http kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    if (e->timing_on) { CUDA_TRY(cudaEventRecord(ev1, st)); e->timing.emplace_back(ev0, ev1); }
-    e->launches++;
-    return GOFR_OK;
+    const int grid = (int)std::min<uint32_t>((uint32_t)e->http_grid, p.n_tiles);
+    return run_launch(e, "http", true, st, [&] { return launch_http_parse(p, grid, st); });
 }
 
 int gofr_requestlog_device(gofr_engine* e, const gofr_log_desc* d_desc, const uint8_t* d_trace_ids, const uint8_t* d_arena,
@@ -1296,37 +1194,12 @@ int gofr_requestlog_device(gofr_engine* e, const gofr_log_desc* d_desc, const ui
     std::lock_guard<std::mutex> g(e->mu);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (n == 0) { if (d_out_off) CUDA_TRY(cudaMemsetAsync(d_out_off, 0, 4, st)); return GOFR_OK; }
-    size_t tiles = (n + kServeThreads - 1) / kServeThreads;
-    if (tiles > e->state_tiles) {
-        cudaFree(e->d_state);
-        e->d_state = nullptr;
-        CUDA_TRY(cudaMalloc(&e->d_state, tiles * 8));
-        CUDA_TRY(cudaMemset(e->d_state, 0, tiles * 8));
-        e->state_tiles = tiles;
-    }
-    if (e->reqlog_grid <= 0) {
-        e->reqlog_grid = reqlog_max_grid(e->device);
-        if (e->reqlog_grid <= 0) { set_last_error("request-log kernel cannot be resident"); return GOFR_ERR_CUDA; }
-    }
     LogParams p;
-    memset(&p, 0, sizeof p);
-    p.desc = d_desc; p.ids = d_trace_ids; p.arena = d_arena; p.n = n; p.n_tiles = (uint32_t)tiles;
-    { int erc = next_epoch(e, &p.epoch); if (erc) return erc; }
-    p.out = d_out; p.out_cap = out_cap; p.out_off = d_out_off;
-    p.tile_state = e->d_state; p.overflow = e->d_flag;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (e->timing_on) {
-        fold_timing(e);
-        CUDA_TRY(cudaEventCreate(&ev0));
-        CUDA_TRY(cudaEventCreate(&ev1));
-        CUDA_TRY(cudaEventRecord(ev0, st));
-    }
-    int rc = launch_reqlog(p, (int)std::min<size_t>((size_t)std::max(1, e->reqlog_grid / engines_on_device(e->device)), tiles), st);
-    if (rc != 0) { set_last_error("request-log kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc)); return GOFR_ERR_CUDA; }
-    if (e->timing_on) { CUDA_TRY(cudaEventRecord(ev1, st)); e->timing.emplace_back(ev0, ev1); }
-    e->launches++;
-    return GOFR_OK;
+    { int rc = frame_prologue(e, n, d_out, out_cap, d_out_off, st, &p); if (rc || n == 0) return rc; }
+    { int rc = lazy_grid(e, &e->reqlog_grid, reqlog_max_grid, "request-log"); if (rc) return rc; }
+    p.desc = d_desc; p.ids = d_trace_ids; p.arena = d_arena;
+    const int grid = lookback_grid(e, e->reqlog_grid, p.n_tiles);
+    return run_launch(e, "request-log", true, st, [&] { return launch_reqlog(p, grid, st); });
 }
 
 }  // extern "C"

@@ -60,9 +60,6 @@ constexpr int kServeCtasWide = GOFR_SERVE_CTAS_WIDE;  // slot layout, "wide" ins
 template <typename Header>
 inline uint32_t image_data_expand(const Header& H) { return H.reserved3[0] > 6u ? H.reserved3[0] : 6u; }
 
-// table_build.cpp: which slot-layout instance suits the sealed table (engine.cu choose_slot_residency)
-bool image_wants_wide_slots(const uint8_t* image);
-
 // Returns dynamic shared memory bytes needed for the table's hot part plus the request-byte staging area.
 uint32_t serve_smem_bytes(uint32_t hot_bytes, uint32_t in_cap);
 // cudaError_t as int
@@ -71,6 +68,27 @@ int launch_serve(const ServeParams& p, int grid, uint32_t smem_bytes, void* stre
 // dynamic shared memory, and the largest per-request staging budget that keeps `ctas` CTAs of the group resident
 int serve_max_grid(uint32_t smem_bytes, int device, int* blocks_per_sm, bool wide);
 uint32_t serve_fit_in_per(uint32_t hot_bytes, int ctas, bool wide);
+
+#if defined(__CUDACC__)
+// Host-side occupancy questions about a kernel of the translation unit that asks; -1 when the runtime cannot answer.
+// Grid of a persistent kernel: CTAs of `threads` threads and `smem_bytes` of dynamic shared memory resident at once.
+template <typename Kernel>
+int occupancy_grid(Kernel kernel, int threads, size_t smem_bytes, int device) {
+    cudaDeviceProp prop;
+    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
+    int nb = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, threads, smem_bytes) != cudaSuccess) return -1;
+    return nb * prop.multiProcessorCount;
+}
+// CTAs per SM once the kernel is allowed `smem_bytes` of dynamic shared memory.
+template <typename Kernel>
+int occupancy_blocks_per_sm(Kernel kernel, int threads, size_t smem_bytes) {
+    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) return -1;
+    int nb = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, threads, smem_bytes) != cudaSuccess) return -1;
+    return nb;
+}
+#endif
 
 // egress of the host-batch path (egress_kernel.cu)
 struct ChunkInfo {

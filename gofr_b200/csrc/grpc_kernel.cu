@@ -59,33 +59,15 @@ int launch_proto_decode(const GrpcParams& p, const ProtoSchema& S, int grid, voi
     return (int)cudaGetLastError();
 }
 
-int proto_decode_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, proto_decode_kernel, GT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int proto_decode_max_grid(int device) { return occupancy_grid(proto_decode_kernel, GT, 0, device); }
 
 int launch_proto_encode(const GrpcParams& p, const ProtoSchema& S, int grid, void* stream) {
     proto_encode_kernel<<<grid, GT, 0, (cudaStream_t)stream>>>(p, S);
     return (int)cudaGetLastError();
 }
 
-int proto_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, proto_encode_kernel, GT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int proto_max_grid(int device) { return occupancy_grid(proto_encode_kernel, GT, 0, device); }
 
-int grpc_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, grpc_hello_kernel, GT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int grpc_max_grid(int device) { return occupancy_grid(grpc_hello_kernel, GT, 0, device); }
 
 }  // namespace gofr

@@ -70,12 +70,6 @@ int launch_http_parse(const HttpParams& p, int grid, void* stream) {
     return (int)cudaGetLastError();
 }
 
-int http_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, http_parse_kernel, HT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int http_max_grid(int device) { return occupancy_grid(http_parse_kernel, HT, 0, device); }
 
 }  // namespace gofr

@@ -25,12 +25,6 @@ int launch_proto_decode_nested(const GrpcParams& p, const PbnDesc& D, int grid, 
     return (int)cudaGetLastError();
 }
 
-int proto_nested_decode_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, proto_decode_nested_kernel, GT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int proto_nested_decode_max_grid(int device) { return occupancy_grid(proto_decode_nested_kernel, GT, 0, device); }
 
 }  // namespace gofr

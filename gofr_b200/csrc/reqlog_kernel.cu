@@ -127,12 +127,6 @@ int launch_reqlog(const LogParams& p, int grid, void* stream) {
     return (int)cudaGetLastError();
 }
 
-int reqlog_max_grid(int device) {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, reqlog_kernel, LT, 0) != cudaSuccess) return -1;
-    return nb * prop.multiProcessorCount;
-}
+int reqlog_max_grid(int device) { return occupancy_grid(reqlog_kernel, LT, 0, device); }
 
 }  // namespace gofr

@@ -27,9 +27,8 @@ uint32_t serve_smem_bytes(uint32_t hot_bytes, uint32_t in_cap) {
 // the kernel once and the "5-CTA" instances silently ran 4 per SM.
 int serve_blocks_per_sm(uint32_t smem_bytes, bool wide) {
     if (wide) return serve_slots_blocks_per_sm(smem_bytes, true);
-    if (cudaFuncSetAttribute(serve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, serve_kernel, T, smem_bytes) != cudaSuccess) return -1;
+    int nb = occupancy_blocks_per_sm(serve_kernel, T, smem_bytes);
+    if (nb < 0) return -1;
     const int nb2 = serve_slots_blocks_per_sm(smem_bytes, false);
     const int nbv = serve_values_blocks_per_sm(smem_bytes);
     if (nb2 < 0 || nbv < 0) return -1;

@@ -24,9 +24,8 @@ int serve_slots_blocks_per_sm(uint32_t smem_bytes, bool wide) {
     if (wide) return serve_slots_wide_blocks_per_sm(smem_bytes);
     const int nv = serve_slots_values_blocks_per_sm(smem_bytes);
     if (nv < 0) return -1;
-    if (cudaFuncSetAttribute(serve_slots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, serve_slots_kernel, T, smem_bytes) != cudaSuccess) return -1;
+    const int nb = occupancy_blocks_per_sm(serve_slots_kernel, T, smem_bytes);
+    if (nb < 0) return -1;
     return nb < nv ? nb : nv;
 }
 

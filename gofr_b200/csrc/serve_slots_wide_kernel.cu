@@ -7,12 +7,7 @@ namespace gofr {
 
 __global__ void __launch_bounds__(T, kServeCtasWide) serve_slots_kernel_wide(const __grid_constant__ ServeParams p) { serve_body<true>(p); }
 
-int serve_slots_wide_blocks_per_sm(uint32_t smem_bytes) {
-    if (cudaFuncSetAttribute(serve_slots_kernel_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, serve_slots_kernel_wide, T, smem_bytes) != cudaSuccess) return -1;
-    return nb;
-}
+int serve_slots_wide_blocks_per_sm(uint32_t smem_bytes) { return occupancy_blocks_per_sm(serve_slots_kernel_wide, T, smem_bytes); }
 
 int launch_serve_slots_wide(const ServeParams& p, int grid, uint32_t smem_bytes, void* stream) {
     serve_slots_kernel_wide<<<grid, T, smem_bytes, (cudaStream_t)stream>>>(p);

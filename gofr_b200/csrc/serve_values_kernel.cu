@@ -7,12 +7,7 @@ namespace gofr {
 
 __global__ void __launch_bounds__(T, kServeCtas) serve_kernel_values(const __grid_constant__ ServeParams p) { serve_body<false>(p); }
 
-int serve_values_blocks_per_sm(uint32_t smem_bytes) {
-    if (cudaFuncSetAttribute(serve_kernel_values, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess) return -1;
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, serve_kernel_values, T, smem_bytes) != cudaSuccess) return -1;
-    return nb;
-}
+int serve_values_blocks_per_sm(uint32_t smem_bytes) { return occupancy_blocks_per_sm(serve_kernel_values, T, smem_bytes); }
 
 int launch_serve_values(const ServeParams& p, int grid, uint32_t smem_bytes, void* stream) {
     serve_kernel_values<<<grid, T, smem_bytes, (cudaStream_t)stream>>>(p);

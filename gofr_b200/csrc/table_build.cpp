@@ -691,31 +691,6 @@ struct Builder {
 
 namespace gofr {
 
-// The tables the wide slot-layout instance (serve_slots_wide_kernel.cu: 4 CTAs/SM, 128 registers) was meant for: every live
-// route answers through the template fast path with ONE program shape and no Bind — warps never diverge between programs
-// and the general pass after the tile loop only sees the odd escaped string.  Informational since the end of round 2: the
-// 5-CTA instance is the faster one even there (engine.cu choose_slot_residency).
-bool image_wants_wide_slots(const uint8_t* img) {
-    const ImageHeader& H = *reinterpret_cast<const ImageHeader*>(img);
-    const RouteRec* routes = reinterpret_cast<const RouteRec*>(img + H.routes_off);
-    const ProgRec* progs = reinterpret_cast<const ProgRec*>(img + H.progs_off);
-    const FastRec* fast = reinterpret_cast<const FastRec*>(img + H.fast_off);
-    int shape = -1;
-    for (uint32_t r = 0; r < H.n_routes; r++) {
-        const RouteRec& R = routes[r];
-        // the routes App.Run appends (health, favicon, catch-all) are not what an application's traffic looks like
-        if (R.flags & (RF_DEAD | RF_DEFAULT)) continue;
-        if (R.prog_ok == 0xFFFF) return false;  // host handlers: the kernel only routes
-        const ProgRec& P = progs[R.prog_ok];
-        if (!(P.flags & PF_FAST) || (P.flags & PF_BIND)) return false;
-        if (fast[R.prog_ok].flags & FR_COMPLETE) continue;  // template only: nothing is interpreted
-        if (shape >= 0 && shape != P.shape_class) return false;
-        shape = P.shape_class;
-    }
-    return shape >= 0;
-}
-
-
 struct Pool {
     std::vector<uint8_t>& img;
     std::map<std::string, uint32_t> seen;
